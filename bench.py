@@ -2,6 +2,7 @@
 """bench.py — camera frames/s @1080p multi-task on B200 (BASELINE.json metric), one JSON line.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py --steps K --dump-outputs DIR   # also write the last timed step's outputs (dump_outputs)
     python bench.py --autospeed ...      # row f.4: the AutoSpeed detector, 1080p frame -> boxes
     python bench.py --config5 ...        # row e: multi-camera all-gather + fusion, one rank per camera (torchrun)
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
@@ -198,6 +199,19 @@ def make_checkpoints(tmpdir: str):
     return paths, sds
 
 
+def dump_outputs(eng, out_dir):
+    """What the engine's last frame returned to its caller, as float32 .npy files (6 MB in all):
+    <model>_raw.npy = the fp32 NCHW tensor (logits, depth, lane masks), <model>_cls.npy = the class / mask map
+    (absent for Scene3D)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for i, m in enumerate(MODELS):
+        eng.fetch_raw(i)                   # D2H on the engine's stream, after that frame, then a sync
+        np.save(os.path.join(out_dir, f"{m}_raw.npy"), eng.raw(i).astype(np.float32))
+        cls = eng.cls(i)
+        if cls is not None:
+            np.save(os.path.join(out_dir, f"{m}_cls.npy"), cls.astype(np.float32))
+
+
 def cpu_reference_frame(sds, frame):
     """The reference's CPU path for one frame, multi-task the way the reference runs it (one
     helper per model, nothing shared): PIL bicubic resize -> ToTensor/Normalize -> network ->
@@ -301,17 +315,7 @@ def run_config5(args, rank, local_rank, world):
     for i in range(max(args.warmup, 3)):
         step(i)
     torch.cuda.synchronize()
-    t_est = time.time()
-    for i in range(args.steps):
-        step(i)
-    torch.cuda.synchronize()
-    t_est = time.time() - t_est
-    blocks = max(1, int(np.ceil(args.min_seconds / max(t_est, 1e-4))))
-    if world > 1:
-        tb = torch.tensor([blocks], device=dev)
-        dist.all_reduce(tb, op=dist.ReduceOp.MAX)
-        blocks = int(tb.item())
-    timed_steps = blocks * args.steps
+    timed_steps = args.steps
     sampler = ClockSampler(local_rank)
     sampler.start()
     barrier()
@@ -382,16 +386,7 @@ def run_autospeed(args, rank, local_rank, world):
     for i in range(max(args.warmup, 3)):
         step(i)
     torch.cuda.synchronize()
-    t_est = time.time()
-    for i in range(args.steps):
-        step(i)
-    torch.cuda.synchronize()
-    blocks = max(1, int(np.ceil(args.min_seconds / max(time.time() - t_est, 1e-4))))
-    if world > 1:
-        tb = torch.tensor([blocks], device=dev)
-        dist.all_reduce(tb, op=dist.ReduceOp.MAX)
-        blocks = int(tb.item())
-    timed_steps = blocks * args.steps
+    timed_steps = args.steps
     sampler = ClockSampler(local_rank)
     sampler.start()
     barrier()
@@ -459,12 +454,17 @@ def main():
                     help="BASELINE configs[4]: per rank EgoLanes + device lateral post-process, ONE ncclAllGather of the "
                          "fused features + PathFinder measurements (C++, vp_b200_multicam.h), Estimator fusion")
     ap.add_argument("--autospeed", action="store_true", help="SURVEY 8f.4: the AutoSpeed detector instead of the 4-task frame")
-    ap.add_argument("--min-seconds", type=float, default=1.0,
-                    help="the K-step block is repeated inside the timed region until it lasts at least this long")
     ap.add_argument("--inflight", type=int, default=4,
                     help="camera frames in flight per GPU (engine replicas on separate streams; the next "
                          "frame's latency-bound encoder overlaps the current frame's decoders)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (every model's fp32 tensor and "
+                         "class / mask map) as DIR/<model>_{raw,cls}.npy, float32; the multi-task benchmark only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.autospeed or args.config5):
+        ap.error("--dump-outputs applies to the multi-task benchmark only")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -525,19 +525,7 @@ def main():
     for i in range(max(args.warmup, 2 * n_eng)):
         step(i)
     torch.cuda.synchronize()
-    # minimum timed duration: one untimed K-step block gives the estimate, the timed region then repeats the
-    # K-step block `blocks` times back to back (a 20-step region is 33 ms — too short to be a measurement)
-    t_est = time.time()
-    for i in range(args.steps):
-        step(i)
-    torch.cuda.synchronize()
-    t_est = time.time() - t_est
-    blocks = max(1, int(np.ceil(args.min_seconds / max(t_est, 1e-4))))
-    if world > 1:
-        tb = torch.tensor([blocks], device="cuda")
-        dist.all_reduce(tb, op=dist.ReduceOp.MAX)
-        blocks = int(tb.item())
-    timed_steps = blocks * args.steps
+    timed_steps = args.steps
 
     sampler = ClockSampler(local_rank)
     sampler.start()
@@ -557,6 +545,9 @@ def main():
     ms = elapsed_all(e0, ends)
     ms = multicam.max_over_ranks(ms, torch.device("cuda", local_rank))
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # before the end-to-end runs below overwrite the engines' outputs
+        dump_outputs(engs[(timed_steps - 1) % n_eng], args.dump_outputs)
 
     # ---- end to end through the C-ABI with pinned host frames (H2D + kernels + D2H per step)
     # (a) latency: one engine, synchronous per frame
@@ -641,8 +632,7 @@ def main():
         "metric": "camera frames/sec @1080p multi-task", "value": fps, "unit": "frames/s", "n_gpus": world,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms / timed_steps, "higher_is_better": True,
         "timed_steps": timed_steps, "timed_region_s": ms / 1e3,
-        "timing": f"the {args.steps}-step block repeated {blocks}x back to back inside ONE device-timed region "
-                  f"(>= {args.min_seconds} s), max over ranks",
+        "timing": f"{timed_steps} steps back to back inside ONE device-timed region, max over ranks",
         "scaling": "weak", "vs_baseline": None, "dtype": "f16" if args.dtype == "fp16" else "bf16",
         "data": "synthetic",
         "config": {"workload": "1080p multi-task: SceneSeg+Scene3D+DomainSeg+EgoLanes, shared encoder "

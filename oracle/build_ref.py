@@ -1,5 +1,5 @@
 """TEST INFRASTRUCTURE ONLY — recipe that compiles the reference's own lateral post-process sources, where
-they lie under /root/reference, into oracle/_ref/libref_lateral.so (git-ignored):
+they lie under ref_import.REFERENCE_ROOT, into oracle/_ref/libref_lateral.so (git-ignored):
 
   g++ -O2 -ffp-contract=off -shared -fPIC  -I oracle/cvstub  -I <ref>/include
       oracle/ref_lateral_harness.cpp  <ref>/src/lane_filtering/lane_filter.cpp
@@ -7,15 +7,17 @@ they lie under /root/reference, into oracle/_ref/libref_lateral.so (git-ignored)
 
 The reference's build system (cmake + OpenCV + Eigen + TensorRT) is NOT run; the OpenCV and Eigen names these five
 files use are provided by the minimal stand-ins oracle/cvstub/opencv2/opencv.hpp and oracle/cvstub/Eigen/Dense.
-Returns the path of the library, or None when /root/reference is absent (GPU box) or the compile fails."""
+Returns the path of the library, or None when the reference sources are absent or the compile fails."""
 from __future__ import annotations
 
 import os
 import subprocess
 from typing import Optional
 
+from oracle import ref_import
+
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference/VisionPilot/production_release"
+REF = os.path.join(ref_import.REFERENCE_ROOT, "VisionPilot", "production_release")
 OUT = os.path.join(HERE, "_ref", "libref_lateral.so")
 
 

@@ -45,10 +45,10 @@ def main():
         smalls[i] = small
         Image.fromarray(small).save(os.path.join(OUT, f"frame_{i:02d}.png"), optimize=True)
     Image.fromarray(frames[FULL_RES]).save(os.path.join(OUT, f"frame_{FULL_RES:02d}_1080p.png"), optimize=True)
-    torch.set_num_threads(os.cpu_count())
+    torch.set_num_threads(8)            # tests/test_oracle_real_images.py evaluates the oracle with the same count
     for m in net.MODELS:
         ref = ref_import.build_network(m, synth.synth_state_dict(m))
-        rec = {}
+        rec = {"threads": np.int64(torch.get_num_threads())}     # the count the goldens were computed with
         for i, small in smalls.items():
             with torch.no_grad():
                 o = ref(net.to_tensor_normalize(small))
